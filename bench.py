@@ -2,6 +2,7 @@
 """bench.py — RGBD frames/s integrated (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C2|C3|C4|C5]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] (C2: TUM1-shape 640x480, 5 mm voxels, tau 0.04 m, 300 synthetic frames
 per step).  `--config C3` (Replica shape 1200x680 + class labels), `C4` (ScanNet shape, 4 mm, meant for 4 GPUs) and
@@ -334,6 +335,26 @@ def shard_checksum(dump):
     return total, len(dump["keys"])
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, vol, suffix="", budget=DUMP_BYTES):
+    """What a caller reads back from the volume after the last timed step, as .npy files in out_dir: the block count,
+    and block keys (float64 [m,3]) with their tsdf, weight (float32 [m,512]) and rgb (float32 [m,3,512]) planes,
+    sorted by key.  When all blocks would exceed `budget` bytes, m is a fixed seeded sample of them."""
+    d = vol.dump_blocks()
+    keys, vox = d["keys"], d["vox"]
+    order = np.lexsort((keys[:, 2], keys[:, 1], keys[:, 0]))
+    m = min(len(order), budget // (3 * 8 + vox.itemsize * int(np.prod(vox.shape[1:]))))
+    if m < len(order):
+        order = order[np.sort(np.random.default_rng(0).choice(len(order), m, replace=False))]
+    keys, vox = keys[order], vox[order]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("num_blocks", np.array([len(d["keys"])], np.float64)), ("block_keys", keys.astype(np.float64)),
+                    ("tsdf", vox[:, 0]), ("weight", vox[:, 1]), ("rgb", vox[:, 2:5])):
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.ascontiguousarray(a))
+
+
 def run_gpu_arm(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -389,10 +410,19 @@ def run_gpu_arm(args, rank, world, local_rank):
         ingest.synchronize()
         return vol.last_frame_stats()  # D2H read of the step's result (the volume's counter block)
 
-    # ---- warm-up (populates the map: steady state afterwards); the clock sampler starts here so that it is up
-    #      (nvidia-smi takes ~0.2 s to deliver its first sample) when the timed regions run ----
+    # ---- the clock sampler starts first so that it is up (nvidia-smi takes ~0.2 s to deliver its first sample)
+    #      when the timed regions run; the GPU stays under load until it delivers ----
     sampler = ClockSampler(local_rank)
     sampler.start()
+    t_load = time.perf_counter()
+    while len(sampler.rows) < 2 and time.perf_counter() - t_load < 1.5:
+        step_resident()
+        torch.cuda.synchronize()
+    # the loop above runs a varying number of steps: start the map again so that every run integrates the same
+    # number of passes before the timed region ends (the outputs of --dump-outputs are then reproducible)
+    vol.reset()
+
+    # ---- warm-up (populates the map: steady state afterwards) ----
     for _ in range(max(args.warmup, 3)):
         step_resident()
     torch.cuda.synchronize()
@@ -402,10 +432,6 @@ def run_gpu_arm(args, rank, world, local_rank):
     # ---- value: inputs resident in HBM, CUDA events on the launching stream ----
     barrier()
     torch.cuda.synchronize()
-    t_load = time.perf_counter()
-    while len(sampler.rows) < 2 and time.perf_counter() - t_load < 1.5:   # under load until the sampler delivers
-        step_resident()
-        torch.cuda.synchronize()
     for _ in range(2):
         step_resident()
     torch.cuda.synchronize()
@@ -421,6 +447,9 @@ def run_gpu_arm(args, rank, world, local_rank):
     ms_max = all_max(e0.elapsed_time(e1))
     upd1, launches1 = vol.counters()
     value = args.steps * F / (ms_max * 1e-3)
+    if args.dump_outputs:
+        # every rank writes its own shard: the 64 MB are shared out among the ranks
+        dump_outputs(args.dump_outputs, vol, f"_rank{rank}" if world > 1 else "", DUMP_BYTES // world)
 
     # ---- e2e: pinned host frames through the public API, H2D (+ NVLink all-gather) inside the timed region ----
     for _ in range(2):
@@ -726,7 +755,13 @@ def main():
     ap.add_argument("--shard-of", type=int, default=0,
                     help="diagnostic (N=1 only): act as rank 0 of a --shard-of-way sharded job on one GPU; ranks share "
                          "nothing, so this is the per-rank work of that job")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the volume they built to DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU volume; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

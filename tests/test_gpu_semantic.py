@@ -15,7 +15,7 @@ import pytest
 import oracle
 from pyslam_b200 import (VoxelBlockSemanticGrid, VoxelBlockSemanticProbabilisticGrid, VoxelSemanticGrid,
                          VoxelSemanticGridProbabilistic)
-from tests._util import GOLDEN, sort_dump
+from tests._util import GOLDEN, SEGMENT_QUERIES, feed_segment_blobs, golden_segments, segment_blobs, sort_dump
 
 pytestmark = pytest.mark.gpu
 
@@ -412,49 +412,36 @@ def test_spatial_read_outs_match_the_compiled_reference(tag):
 @pytest.mark.parametrize("kind", ["voting", "probabilistic"])
 def test_object_and_class_segments_and_integrate_segment_match_the_reference(kind):
     """get_object_segments / get_class_segments / integrate_segment (voxel_block_semantic_grid.hpp:52-99, 204-316)
-    against the UNMODIFIED compiled reference: same segment ids, the same voxels (positions, colours) in every
-    segment, class ids, confidence ranges; PCA boxes to 1e-9."""
+    against the stored segments of the same stream (tests/golden/segments_T0.npz; its `source` says what recorded it,
+    and test_oracle_semantic.py::test_compiled_reference_reproduces_the_segment_goldens compares it with the
+    UNMODIFIED compiled reference at these tolerances): same segment ids, the same voxels (positions, colours) in
+    every segment, class ids, confidence ranges; PCA boxes to 1e-9."""
     from pyslam_b200 import VoxelBlockSemanticGrid, VoxelBlockSemanticProbabilisticGrid
-    rng = np.random.default_rng(3)
+    ref = np.load(os.path.join(GOLDEN, "segments_T0.npz"))
+    tag = "vote" if kind == "voting" else "prob"
     Cls = VoxelBlockSemanticGrid if kind == "voting" else VoxelBlockSemanticProbabilisticGrid
-    g = Cls(0.05, 8, capacity_blocks=1 << 13)
-    r = oracle.RefSemanticGrid(0.05, kind)
-    blobs = []
-    for oid, (c, sc) in enumerate([((0, 0, 1), (0.5, 0.2, 0.1)), ((2, 1, 1), (0.1, 0.6, 0.3)), ((-1, 2, 0.5), (0.3, 0.3, 0.3))], 1):
-        Q, _ = np.linalg.qr(rng.normal(size=(3, 3)))
-        blobs.append((oid, oid + 10, (rng.normal(size=(3000, 3)) * np.array(sc)) @ Q.T + np.array(c),
-                      rng.random((3000, 3)).astype(np.float32)))
-    for rep in range(3):
-        for oid, cid, p, col in blobs:
-            if rep == 1:   # the per-segment entry point
-                g.integrate_segment(p, col, cid, oid)
-                r.integrate_segment(p, col, cid, oid)
-            else:
-                ids_c, ids_o = np.full(len(p), cid, np.int32), np.full(len(p), oid, np.int32)
-                g.integrate(p, col, ids_c, ids_o)
-                r.integrate(p, col, ids_c, ids_o)
-    g.integrate_segment(blobs[0][2], blobs[0][3], -1, 5)      # a negative id skips the whole segment
-    r.integrate_segment(blobs[0][2], blobs[0][3], -1, 5)
+    g = Cls(float(ref["voxel_size"]), 8, capacity_blocks=1 << 13)
+    blobs = segment_blobs(np.random.default_rng(3), 3000)
+    feed_segment_blobs(g, blobs)
     with pytest.raises(RuntimeError):
         g.integrate_segment(blobs[0][2], blobs[0][3][:5], 1, 1)
-    for by_class in (False, True):
-        for min_count, min_conf in ((1, 0.0), (2, 0.5)):
-            a = (g.get_class_segments if by_class else g.get_object_segments)(min_count, min_conf)
-            b = (r.get_class_segments if by_class else r.get_object_segments)(min_count, min_conf)
-            av = a.class_vector if by_class else a.object_vector
-            ids_a = [x.class_id if by_class else x.object_id for x in av]
-            assert sorted(ids_a) == sorted(s["id"] for s in b) and len(b) == 3
-            for x in av:
-                s = next(s for s in b if s["id"] == (x.class_id if by_class else x.object_id))
-                oa = np.lexsort(np.asarray(x.points).T[::-1])
-                ob = np.lexsort(s["points"].T[::-1])
-                assert np.array_equal(np.asarray(x.points)[oa], s["points"][ob])       # float64 means, bit for bit
-                assert np.allclose(np.asarray(x.colors)[oa], s["colors"][ob], rtol=0, atol=1e-6)
-                assert abs(x.confidence_min - s["confidence_min"]) < 1e-5
-                assert abs(x.confidence_max - s["confidence_max"]) < 1e-5
-                if not by_class:
-                    assert x.class_id == s["class_id"]
-                    box = x.oriented_bounding_box
-                    assert np.abs(box.center - s["obb_center"]).max() < 1e-9
-                    assert np.abs(box.size - s["obb_size"]).max() < 1e-9
+    for query, (by_class, min_count, min_conf) in enumerate(SEGMENT_QUERIES):
+        a = (g.get_class_segments if by_class else g.get_object_segments)(min_count, min_conf)
+        b = golden_segments(ref, tag, query)
+        av = a.class_vector if by_class else a.object_vector
+        ids_a = [x.class_id if by_class else x.object_id for x in av]
+        assert sorted(ids_a) == sorted(s["id"] for s in b) and len(b) == 3
+        for x in av:
+            s = next(s for s in b if s["id"] == (x.class_id if by_class else x.object_id))
+            oa = np.lexsort(np.asarray(x.points).T[::-1])
+            ob = np.lexsort(s["points"].T[::-1])
+            assert np.array_equal(np.asarray(x.points)[oa], s["points"][ob])       # float64 means, bit for bit
+            assert np.allclose(np.asarray(x.colors)[oa], s["colors"][ob], rtol=0, atol=1e-6)
+            assert abs(x.confidence_min - s["confidence_min"]) < 1e-5
+            assert abs(x.confidence_max - s["confidence_max"]) < 1e-5
+            if not by_class:
+                assert x.class_id == s["class_id"]
+                box = x.oriented_bounding_box
+                assert np.abs(box.center - s["obb_center"]).max() < 1e-9
+                assert np.abs(box.size - s["obb_size"]).max() < 1e-9
     g.close()
