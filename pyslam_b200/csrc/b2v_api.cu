@@ -8,8 +8,6 @@
 // frame f.  Nothing synchronises with the host until b2v_synchronize / an inspection call.
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <string>
@@ -99,6 +97,22 @@ bool is_device_pointer(const void *p) {
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
+// Depth images of an integrate call: float32 metres (u16_scale == 0) or raw uint16 that the device widens to
+// float(depth) * u16_scale.
+struct DepthInput {
+    const void *ptr;
+    float u16_scale;
+};
+
+// The images of one integrate call: frames of H x W pixels back to back, each kind on the host (staged through the
+// copy stream) or on the device (read in place).
+struct FrameImages {
+    DepthInput depth;
+    const uint8_t *color;
+    int32_t H, W;
+    bool dev_depth, dev_color;
+};
+
 }  // namespace
 
 struct b2v_volume {
@@ -107,7 +121,6 @@ struct b2v_volume {
     cudaStream_t compute = nullptr, copy = nullptr, alloc = nullptr;
     cudaStream_t last_stream = nullptr;  // caller stream of the most recent frame (synchronised on reads)
     bool overlap = true;                 // allocate(f+1) on its own stream, concurrent with integrate(f)
-    bool use_tma = true;                 // stage image tiles with TMA when the layout allows it
     bool inputs_fenced = false;          // batch call: device inputs already ordered before the alloc stream
     bool fuse = true;                    // b2v_integrate_batch fuses groups of up to kMaxGroup frames
     int group_frames = 16;               // frames per fused group (1..kMaxGroup), b2v_set_group_size
@@ -115,8 +128,6 @@ struct b2v_volume {
     bool lam_map_ok = false;
     cudaEvent_t input_event = nullptr;   // b2v_set_input_event: readiness of the next batch's device inputs
     bool rings_stale = false;            // a fused batch advanced frame_id: the per-frame ring counters must be re-armed
-    float4 *d_gtex[kGroupBufs * kMaxGroup] = {};  // texel images of the group buffers
-    size_t gtex_pixels = 0;
     uint32_t group_id = 0;
     cudaEvent_t ev_galloc[kGroupBufs] = {}, ev_group_done[kGroupBufs] = {};
     int last_group_buf = -1, last_group_count = 0;  // most recent frame came from a fused group
@@ -124,24 +135,25 @@ struct b2v_volume {
     // optional rectification stage (b2v_set_rectification)
     float *d_mapx = nullptr, *d_mapy = nullptr;
     int rect_H = 0, rect_W = 0, rect_swap = 0;
-    float *d_rdepth[kStage] = {};    // rectified frames (same slot layout as the raw staging)
-    uint8_t *d_rcolor[kStage] = {};
     // TMA descriptors are cached per image address (encoding costs ~1 us of host time each)
     std::unordered_map<uintptr_t, FrameMaps> map_cache;
     int map_H = 0, map_W = 0;
     const float *map_lam = nullptr;
     cudaEvent_t ev_in = nullptr, ev_alloc_done[kActiveRing] = {}, ev_int_done[kActiveRing] = {};
-    // raw 16-bit depth input (b2v_integrate_u16 / b2v_integrate_batch_u16): uploaded as is, widened on the device
-    uint16_t *d_depth16[kStage] = {};   // same slot layout as d_depth; allocated on first use
-    size_t stage16_pixels = 0;
-    float in_u16_scale = 0.0f;          // > 0 while a *_u16 entry point runs: `depth` pointers are uint16_t
-    float *d_depth[kStage] = {};
-    uint8_t *d_color[kStage] = {};
-    float4 *d_texel[kStage] = {};   // packed {depth, lambda, rgbx} frames read by integrate_kernel
+    // Frame staging (ensure_staging): one allocation per image kind, holding slots of stage_pixels pixels.  The
+    // kStage raw and rectified slots are the kGroupStage slots of the group buffers followed by the kFrameStage
+    // slots of the per-frame ring; the texel kinds hold only the slots of their own path.
+    size_t stage_pixels = 0;
+    float *d_depth = nullptr;       // raw float32 depth: host uploads and widened uint16 depth
+    uint8_t *d_color = nullptr;     // raw colour
+    uint16_t *d_depth16 = nullptr;  // raw uint16 depth; allocated on first use
+    float *d_rdepth = nullptr;      // rectified frames; allocated while maps are installed
+    uint8_t *d_rcolor = nullptr;
+    float4 *d_texel = nullptr;      // kFrameStage packed {depth, lambda, rgbx} frames read by integrate_kernel
+    float4 *d_gtex = nullptr;       // kGroupStage texel images of the group buffers; allocated on first use
     float *d_lambda = nullptr;      // lambda image of the cached intrinsics
     double lam_K[4] = {0, 0, 0, 0};
     int lam_H = 0, lam_W = 0;
-    size_t stage_pixels = 0;
     cudaEvent_t ev_ready[kStage] = {}, ev_free[kStage] = {};
     HashTable table{};
     PoolMeta meta{};
@@ -161,6 +173,12 @@ struct b2v_volume {
     bool prof_enabled = false;
     std::vector<cudaEvent_t> prof_events;  // quadruples: allocate begin/end, integrate begin/end
     size_t prof_used = 0;
+
+    // image k of the run of frames staged from slot s0 of `base`: a run starts on a slot boundary and holds its
+    // frames of `pixels` pixels back to back, so it uploads with one copy per image kind
+    template <typename T> T *staged(T *base, int s0, size_t pixels, int k = 0, int channels = 1) const {
+        return base + (stage_pixels * s0 + pixels * k) * channels;
+    }
 };
 
 #define B2V_CUDA(v, call)                                                                  \
@@ -179,6 +197,24 @@ static int volume_clear_device(b2v_volume *v) {
     B2V_CUDA(v, cudaMemsetAsync(v->meta.group_mask, 0, tcap * kGroupBufs * sizeof(uint32_t), v->compute));
     B2V_CUDA(v, cudaMemsetAsync(v->meta.counters, 0, kNumCounters * sizeof(uint32_t), v->compute));
     return B2V_OK;
+}
+
+// frees every staging kind (ensure_staging); the caller has waited for the device
+static void free_staging(b2v_volume *v) {
+    auto release = [](auto *&p) {
+        cudaFree(p);
+        p = nullptr;
+    };
+    release(v->d_depth);
+    release(v->d_color);
+    release(v->d_depth16);
+    release(v->d_rdepth);
+    release(v->d_rcolor);
+    release(v->d_texel);
+    release(v->d_gtex);
+    release(v->d_lambda);
+    v->stage_pixels = 0;
+    v->lam_H = v->lam_W = 0;
 }
 
 extern "C" int b2v_version(void) { return 100; }
@@ -244,13 +280,6 @@ extern "C" int b2v_create(const b2v_config *cfg, b2v_volume **out) {
         B2V_CUDA(v, cudaEventCreateWithFlags(&v->ev_alloc_done[r], cudaEventDisableTiming));
         B2V_CUDA(v, cudaEventCreateWithFlags(&v->ev_int_done[r], cudaEventDisableTiming));
     }
-    if (const char *e = std::getenv("B2V_OVERLAP")) v->overlap = std::atoi(e) != 0;
-    if (const char *e = std::getenv("B2V_TMA")) v->use_tma = std::atoi(e) != 0;
-    if (const char *e = std::getenv("B2V_FUSE")) v->fuse = std::atoi(e) != 0;
-    if (const char *e = std::getenv("B2V_GROUP")) {
-        const int n = std::atoi(e);
-        if (n >= 1 && n <= kMaxGroup) v->group_frames = n;
-    }
     for (int b = 0; b < kGroupBufs; ++b) {
         B2V_CUDA(v, cudaEventCreateWithFlags(&v->ev_galloc[b], cudaEventDisableTiming));
         B2V_CUDA(v, cudaEventCreateWithFlags(&v->ev_group_done[b], cudaEventDisableTiming));
@@ -281,13 +310,8 @@ extern "C" int b2v_create(const b2v_config *cfg, b2v_volume **out) {
     int rc = volume_clear_device(v);
     if (rc != B2V_OK) return rc;
     const int sms = b2v_device_sm_count(cfg->device);
-    // persistent grid: exactly one wave of resident CTAs (B2V_INT_CTAS_PER_SM overrides, for tuning)
-    int per_sm = integrate_max_resident_ctas_per_sm();
-    if (const char *e = std::getenv("B2V_INT_CTAS_PER_SM")) {
-        const int n = std::atoi(e);
-        if (n >= 1 && n <= 32) per_sm = n;
-    }
-    v->grid_ctas = (sms > 0 ? sms : 148) * per_sm;
+    // persistent grid: exactly one wave of resident CTAs
+    v->grid_ctas = (sms > 0 ? sms : 148) * integrate_max_resident_ctas_per_sm();
     v->sm_count = sms;
     B2V_CUDA(v, cudaStreamSynchronize(v->compute));
     return B2V_OK;
@@ -302,20 +326,13 @@ extern "C" int b2v_destroy(b2v_volume *v) {
         if (v->ev_alloc_done[r]) cudaEventDestroy(v->ev_alloc_done[r]);
         if (v->ev_int_done[r]) cudaEventDestroy(v->ev_int_done[r]);
     }
-    cudaFree(v->d_depth[0]);  // slots 1.. point into the same two allocations
-    cudaFree(v->d_color[0]);
     for (int s = 0; s < kStage; ++s) {
-        cudaFree(v->d_texel[s]);
         if (v->ev_ready[s]) cudaEventDestroy(v->ev_ready[s]);
         if (v->ev_free[s]) cudaEventDestroy(v->ev_free[s]);
     }
-    cudaFree(v->d_lambda);
+    free_staging(v);
     cudaFree(v->d_mapx);
     cudaFree(v->d_mapy);
-    cudaFree(v->d_rdepth[0]);
-    cudaFree(v->d_rcolor[0]);
-    cudaFree(v->d_depth16[0]);
-    for (float4 *t : v->d_gtex) cudaFree(t);
     for (int b = 0; b < kGroupBufs; ++b) {
         if (v->ev_galloc[b]) cudaEventDestroy(v->ev_galloc[b]);
         if (v->ev_group_done[b]) cudaEventDestroy(v->ev_group_done[b]);
@@ -393,55 +410,51 @@ extern "C" int b2v_reset(b2v_volume *v) {
     return B2V_OK;
 }
 
-static int ensure_staging(b2v_volume *v, size_t pixels) {
-    if (pixels <= v->stage_pixels) return B2V_OK;
-    B2V_CUDA(v, cudaStreamSynchronize(v->compute));
-    B2V_CUDA(v, cudaStreamSynchronize(v->copy));
-    B2V_CUDA(v, cudaStreamSynchronize(v->alloc));
-    if (v->last_stream) B2V_CUDA(v, cudaStreamSynchronize(v->last_stream));
-    // raw staging slots are carved out of two contiguous allocations, so the frames of a group (which
-    // are contiguous in the caller's arrays) upload with ONE copy per image type
-    cudaFree(v->d_depth[0]);
-    cudaFree(v->d_color[0]);
-    for (int s = 0; s < kStage; ++s) {
-        cudaFree(v->d_texel[s]);
-        v->d_depth[s] = nullptr;
-        v->d_color[s] = nullptr;
-        v->d_texel[s] = nullptr;
+// Allocates the staging kinds that the next frames need, for images of `pixels` pixels: raw depth and colour, the
+// per-frame texels and the lambda image always; raw uint16 depth, the group texels and the rectified frames once a
+// call needs them.  Larger images reallocate every kind.  Kernels on any stream, a caller's stream included, may still
+// read the old buffers, so that waits for the whole device; it happens only when the image size grows.
+static int ensure_staging(b2v_volume *v, size_t pixels, bool u16, bool group) {
+    if (pixels > v->stage_pixels) {
+        B2V_CUDA(v, cudaDeviceSynchronize());
+        free_staging(v);
+        v->stage_pixels = pixels;
     }
-    v->stage_pixels = 0;  // stays 0 if an allocation below fails
-    float *dbase = nullptr;
-    uint8_t *cbase = nullptr;
-    B2V_CUDA(v, cudaMalloc(&dbase, pixels * sizeof(float) * kStage));
-    v->d_depth[0] = dbase;
-    B2V_CUDA(v, cudaMalloc(&cbase, pixels * 3 * kStage));
-    v->d_color[0] = cbase;
-    for (int s = 0; s < kStage; ++s) {
-        v->d_depth[s] = dbase + pixels * s;
-        v->d_color[s] = cbase + pixels * 3 * s;
-        if (s >= kGroupStage)  // texel images of the per-frame path (the group buffers have their own)
-            B2V_CUDA(v, cudaMalloc(&v->d_texel[s], pixels * sizeof(float4)));
+    const size_t n = v->stage_pixels;
+    auto alloc = [](auto *&p, size_t elems) { return p ? cudaSuccess : cudaMalloc(&p, elems * sizeof(*p)); };
+    B2V_CUDA(v, alloc(v->d_depth, n * kStage));
+    B2V_CUDA(v, alloc(v->d_color, n * 3 * kStage));
+    B2V_CUDA(v, alloc(v->d_texel, n * kFrameStage));
+    B2V_CUDA(v, alloc(v->d_lambda, n));
+    if (u16) B2V_CUDA(v, alloc(v->d_depth16, n * kStage));
+    if (group) B2V_CUDA(v, alloc(v->d_gtex, n * kGroupStage));
+    if (v->d_mapx) {
+        B2V_CUDA(v, alloc(v->d_rdepth, n * kStage));
+        B2V_CUDA(v, alloc(v->d_rcolor, n * 3 * kStage));
     }
-    cudaFree(v->d_lambda);
-    v->d_lambda = nullptr;
-    B2V_CUDA(v, cudaMalloc(&v->d_lambda, pixels * sizeof(float)));
-    v->lam_H = v->lam_W = 0;
-    v->stage_pixels = pixels;
     return B2V_OK;
 }
 
-static int grow_profile_events(b2v_volume *v, size_t need) {
-    if (v->prof_used + need > v->prof_events.size()) {
+// The four timing events of one allocate / update launch pair (allocate begin, end, update begin, end) while
+// profiling is on, else nullptr.  `frames`: the frames the pair integrates.
+static int profile_events(b2v_volume *v, int frames, cudaEvent_t **pe) {
+    *pe = nullptr;
+    if (!v->prof_enabled) return B2V_OK;
+    if (v->prof_used + 4 > v->prof_events.size()) {
         const size_t old = v->prof_events.size();
         v->prof_events.resize(old + 4 * 256, nullptr);
         for (size_t k = old; k < v->prof_events.size(); ++k) B2V_CUDA(v, cudaEventCreate(&v->prof_events[k]));
     }
+    *pe = &v->prof_events[v->prof_used];
+    v->prof_used += 4;
+    v->prof_frames += frames;
+    v->prof_int_launches += 1;
     return B2V_OK;
 }
 
 // cached TMA descriptors of a frame (keyed by the depth image address; colour address is checked)
 static const FrameMaps *frame_maps(b2v_volume *v, const float *d_depth, const uint8_t *d_color, int H, int W) {
-    if (!v->use_tma || !tma_tiles_usable(W, v->cfg.depth_stride, d_depth, d_color, v->d_lambda)) return nullptr;
+    if (!tma_tiles_usable(W, v->cfg.depth_stride, d_depth, d_color, v->d_lambda)) return nullptr;
     if (v->map_H != H || v->map_W != W || v->map_lam != v->d_lambda || v->map_cache.size() > 4096) {
         v->map_cache.clear();
         v->map_H = H;
@@ -459,82 +472,112 @@ static const FrameMaps *frame_maps(b2v_volume *v, const float *d_depth, const ui
     return &res.first->second;
 }
 
-static int rectify_frame(b2v_volume *v, const float **d_depth, const uint8_t **d_color, int H, int W, int slot,
-                         cudaStream_t stream);
-
-// raw uint16 staging, one contiguous allocation carved into the same slots as the float staging
-static int ensure_staging16(b2v_volume *v, size_t pixels) {
-    if (pixels <= v->stage16_pixels) return B2V_OK;
-    B2V_CUDA(v, cudaStreamSynchronize(v->compute));
-    B2V_CUDA(v, cudaStreamSynchronize(v->copy));
-    B2V_CUDA(v, cudaStreamSynchronize(v->alloc));
-    if (v->last_stream) B2V_CUDA(v, cudaStreamSynchronize(v->last_stream));
-    cudaFree(v->d_depth16[0]);
-    for (int s = 0; s < kStage; ++s) v->d_depth16[s] = nullptr;
-    v->stage16_pixels = 0;
-    uint16_t *base = nullptr;
-    B2V_CUDA(v, cudaMalloc(&base, pixels * sizeof(uint16_t) * kStage));
-    for (int s = 0; s < kStage; ++s) v->d_depth16[s] = base + pixels * s;
-    v->stage16_pixels = pixels;
+// recomputes the lambda image when the intrinsics or the image size change
+static int refresh_lambda(b2v_volume *v, const FrameParams &P, const double K[4], int H, int W, cudaStream_t as) {
+    if (v->lam_H == H && v->lam_W == W && std::memcmp(v->lam_K, K, sizeof(v->lam_K)) == 0) return B2V_OK;
+    if (v->overlap) {  // the lambda image is read by allocate kernels that may still be in flight
+        B2V_CUDA(v, cudaStreamSynchronize(v->alloc));
+    }
+    B2V_CUDA(v, launch_lambda(P, v->d_lambda, as));
+    std::memcpy(v->lam_K, K, sizeof(v->lam_K));
+    v->lam_H = H;
+    v->lam_W = W;
+    v->launches += 1;
     return B2V_OK;
 }
 
-static int integrate_frame(b2v_volume *v, const float *depth, const uint8_t *color, int32_t height,
-                           int32_t width, const double K[4], const double Tcw[16], void *stream,
-                           int dev_hint = -1) {
-    if (!depth || !color || !K || !Tcw || height <= 0 || width <= 0) {
-        v->err = "b2v_integrate: null pointer or non-positive image size";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    if (!(K[0] > 0.0) || !(K[1] > 0.0)) {
-        v->err = "b2v_integrate: focal lengths must be positive";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    const size_t pixels = static_cast<size_t>(height) * width;
-    bool dev_depth, dev_color;
-    if (dev_hint >= 0) {  // batch call: queried once for the whole batch
-        dev_depth = dev_color = dev_hint != 0;
-    } else {
+// The checks that every integrate entry point makes, reported under the entry point's name `fn`; also finds where
+// the images of `in` live.
+static int check_integrate(b2v_volume *v, const char *fn, bool u16, int32_t n_frames, FrameImages *in,
+                           const double *K, const double *Tcw, void *stream) {
+    const char *why = nullptr;
+    if (u16 && !(in->depth.u16_scale > 0.0f)) {
+        why = "depth_scale must be positive";
+    } else if (n_frames < 0 || in->H <= 0 || in->W <= 0 ||
+               (n_frames > 0 && (!in->depth.ptr || !in->color || !K || !Tcw))) {
+        why = "null pointer, negative frame count or non-positive image size";
+    } else if (n_frames > 0 && !(K[0] > 0.0 && K[1] > 0.0)) {
+        why = "focal lengths must be positive";
+    } else if (n_frames > 0) {
         B2V_CUDA(v, cudaSetDevice(v->cfg.device));
-        dev_depth = is_device_pointer(depth);
-        dev_color = is_device_pointer(color);
+        in->dev_depth = is_device_pointer(in->depth.ptr);
+        in->dev_color = is_device_pointer(in->color);
+        if (stream != nullptr && !(in->dev_depth && in->dev_color))
+            why = "a caller stream requires device image pointers";
     }
-    if (stream != nullptr && !(dev_depth && dev_color)) {
-        v->err = "b2v_integrate: a caller stream requires device image pointers";
+    if (!why) return B2V_OK;
+    v->err = std::string(fn) + ": " + why;
+    return B2V_ERR_INVALID_ARGUMENT;
+}
+
+// Stages `count` consecutive frames of `in`, from frame f0 on, into the run of slots that starts at slot s0, for the
+// allocate stream `as`.  Host images are uploaded on the copy stream, one copy per image kind, once `ev_free` has
+// fired (the previous reader of the run is done); `ev_ready` orders `as` after the uploads.  Raw uint16 depth is
+// widened in one launch, and every frame is rectified while maps are installed.  Returns the device images that the
+// allocate kernels read, one per frame.
+static int prepare_frames(b2v_volume *v, const FrameImages &in, size_t f0, int count, int s0, cudaEvent_t ev_free,
+                          cudaEvent_t ev_ready, cudaStream_t as, const float **d_depth, const uint8_t **d_color) {
+    const size_t pixels = static_cast<size_t>(in.H) * in.W;
+    const float scale = in.depth.u16_scale;
+    const size_t depth_bytes = scale > 0.0f ? sizeof(uint16_t) : sizeof(float);
+    const void *depth = static_cast<const char *>(in.depth.ptr) + pixels * depth_bytes * f0;
+    const uint8_t *color = in.color + pixels * 3 * f0;
+    float *raw_depth = v->staged(v->d_depth, s0, pixels);
+    uint8_t *raw_color = v->staged(v->d_color, s0, pixels, 0, 3);
+    if (!in.dev_depth || !in.dev_color) {
+        B2V_CUDA(v, cudaStreamWaitEvent(v->copy, ev_free, 0));
+        if (!in.dev_depth) {
+            void *dst = scale > 0.0f ? static_cast<void *>(v->staged(v->d_depth16, s0, pixels)) : raw_depth;
+            B2V_CUDA(v, cudaMemcpyAsync(dst, depth, pixels * depth_bytes * count, cudaMemcpyHostToDevice, v->copy));
+            depth = dst;
+        }
+        if (!in.dev_color) {
+            B2V_CUDA(v, cudaMemcpyAsync(raw_color, color, pixels * 3 * count, cudaMemcpyHostToDevice, v->copy));
+            color = raw_color;
+        }
+        B2V_CUDA(v, cudaEventRecord(ev_ready, v->copy));
+        B2V_CUDA(v, cudaStreamWaitEvent(as, ev_ready, 0));
+    }
+    if (scale > 0.0f) {  // widen into the float slots: float(u16) * scale, one rounding
+        B2V_CUDA(v, launch_depth_u16_to_f32(static_cast<const uint16_t *>(depth), raw_depth, pixels * count, scale, as));
+        depth = raw_depth;
+        v->launches += 1;
+    }
+    for (int k = 0; k < count; ++k) {
+        d_depth[k] = static_cast<const float *>(depth) + pixels * k;
+        d_color[k] = color + pixels * 3 * k;
+    }
+    if (!v->d_mapx) return B2V_OK;
+    if (in.H != v->rect_H || in.W != v->rect_W) {
+        v->err = "rectification maps were installed for a different image size";
         return B2V_ERR_INVALID_ARGUMENT;
     }
+    for (int k = 0; k < count; ++k) {
+        float *rdepth = v->staged(v->d_rdepth, s0, pixels, k);
+        uint8_t *rcolor = v->staged(v->d_rcolor, s0, pixels, k, 3);
+        B2V_CUDA(v, launch_remap_b32_nearest(d_depth[k], in.H, in.W, v->d_mapx, v->d_mapy, rdepth, as));
+        B2V_CUDA(v, launch_remap_u8c3_linear(d_color[k], in.H, in.W, v->d_mapx, v->d_mapy, rcolor, v->rect_swap, as));
+        d_depth[k] = rdepth;
+        d_color[k] = rcolor;
+        v->launches += 2;
+    }
+    return B2V_OK;
+}
+
+// frame f of `in` (pose Tcw) through allocate_kernel + integrate_kernel, staged in the per-frame ring of slots
+static int integrate_frame(b2v_volume *v, const FrameImages &in, size_t f, const double K[4], const double Tcw[16],
+                           void *stream) {
     cudaStream_t cs = stream ? static_cast<cudaStream_t>(stream) : v->compute;
     cudaStream_t as = v->overlap ? v->alloc : cs;  // stream of the allocate kernel
     v->last_stream = stream ? cs : nullptr;
     const int s = kGroupStage + static_cast<int>(v->frame_id % kFrameStage);
     const int ring = static_cast<int>(v->frame_id % kActiveRing);
-    const float *d_depth = depth;
-    const uint8_t *d_color = color;
-    const bool staged = !(dev_depth && dev_color);
-    const bool u16 = v->in_u16_scale > 0.0f;  // `depth` is really const uint16_t *
-    {
-        int rc = ensure_staging(v, pixels);
-        if (rc == B2V_OK && u16) rc = ensure_staging16(v, pixels);
-        if (rc != B2V_OK) return rc;
-    }
-    if (staged) {
-        B2V_CUDA(v, cudaStreamWaitEvent(v->copy, v->ev_free[s], 0));
-        if (!dev_depth) {
-            if (u16)
-                B2V_CUDA(v, cudaMemcpyAsync(v->d_depth16[s], depth, pixels * sizeof(uint16_t), cudaMemcpyHostToDevice,
-                                            v->copy));
-            else
-                B2V_CUDA(v, cudaMemcpyAsync(v->d_depth[s], depth, pixels * sizeof(float),
-                                            cudaMemcpyHostToDevice, v->copy));
-            d_depth = v->d_depth[s];
-        }
-        if (!dev_color) {
-            B2V_CUDA(v, cudaMemcpyAsync(v->d_color[s], color, pixels * 3, cudaMemcpyHostToDevice, v->copy));
-            d_color = v->d_color[s];
-        }
-        B2V_CUDA(v, cudaEventRecord(v->ev_ready[s], v->copy));
-        B2V_CUDA(v, cudaStreamWaitEvent(as, v->ev_ready[s], 0));
-    } else if (v->overlap && !v->inputs_fenced) {
+    const size_t pixels = static_cast<size_t>(in.H) * in.W;
+    const bool staged = !(in.dev_depth && in.dev_color);
+    const bool u16 = in.depth.u16_scale > 0.0f;
+    int rc = ensure_staging(v, pixels, u16, false);
+    if (rc != B2V_OK) return rc;
+    if (!staged && v->overlap && !v->inputs_fenced) {
         // device inputs were produced by earlier work on the caller's stream (a batch call fences once:
         // an event recorded now would also wait for the previous frame's integrate kernel)
         B2V_CUDA(v, cudaEventRecord(v->ev_in, cs));
@@ -553,44 +596,25 @@ static int integrate_frame(b2v_volume *v, const float *depth, const uint8_t *col
         // allocate(f) recycles the ring slot / texel buffer last read by integrate(f - 3) .. (f - 4)
         B2V_CUDA(v, cudaStreamWaitEvent(as, v->ev_int_done[(v->frame_id - 3) % kActiveRing], 0));
     }
-    if (u16) {  // widen the raw depth into the float staging slot: float(u16) * scale, one rounding
-        const uint16_t *src = dev_depth ? reinterpret_cast<const uint16_t *>(depth) : v->d_depth16[s];
-        B2V_CUDA(v, launch_depth_u16_to_f32(src, v->d_depth[s], pixels, v->in_u16_scale, as));
-        d_depth = v->d_depth[s];
-        v->launches += 1;
-    }
-    {
-        const int rc = rectify_frame(v, &d_depth, &d_color, height, width, s, as);
-        if (rc != B2V_OK) return rc;
-    }
+    const float *d_depth;
+    const uint8_t *d_color;
+    rc = prepare_frames(v, in, f, 1, s, v->ev_free[s], v->ev_ready[s], as, &d_depth, &d_color);
+    if (rc != B2V_OK) return rc;
     FrameParams P;
-    fill_frame_params(&P, K, Tcw, height, width, v->geo, v->frame_id + 1);
-    if (v->lam_H != height || v->lam_W != width || std::memcmp(v->lam_K, K, sizeof(v->lam_K)) != 0) {
-        if (v->overlap) {  // the lambda image is read by allocate kernels that may still be in flight
-            B2V_CUDA(v, cudaStreamSynchronize(v->alloc));
-        }
-        B2V_CUDA(v, launch_lambda(P, v->d_lambda, as));
-        std::memcpy(v->lam_K, K, sizeof(v->lam_K));
-        v->lam_H = height;
-        v->lam_W = width;
-        v->launches += 1;
-    }
-    cudaEvent_t *pe = nullptr;
-    if (v->prof_enabled) {
-        const int rc = grow_profile_events(v, 4);
-        if (rc != B2V_OK) return rc;
-        pe = &v->prof_events[v->prof_used];
-        v->prof_used += 4;
-        B2V_CUDA(v, cudaEventRecord(pe[0], as));
-    }
-    float4 *tex = v->d_texel[s];
+    fill_frame_params(&P, K, Tcw, in.H, in.W, v->geo, v->frame_id + 1);
+    rc = refresh_lambda(v, P, K, in.H, in.W, as);
+    if (rc != B2V_OK) return rc;
+    cudaEvent_t *pe;
+    rc = profile_events(v, 1, &pe);
+    if (rc != B2V_OK) return rc;
+    if (pe) B2V_CUDA(v, cudaEventRecord(pe[0], as));
+    float4 *tex = v->staged(v->d_texel, s - kGroupStage, pixels);
     P.I.tex = tex;
     B2V_CUDA(v, launch_allocate(P, d_depth, d_color, v->d_lambda, tex, v->table, v->meta, ring,
-                                frame_maps(v, d_depth, d_color, height, width), &v->lam_map, as));
+                                frame_maps(v, d_depth, d_color, in.H, in.W), &v->lam_map, as));
     if (staged || u16) B2V_CUDA(v, cudaEventRecord(v->ev_free[s], as));  // the raw frame is consumed by allocate only
     v->launches += 1;
     v->frame_id += 1;
-    if (v->prof_enabled) v->prof_frames += 1;
     v->last_group_buf = -1;
     if (pe) B2V_CUDA(v, cudaEventRecord(pe[1], as));
     if (v->overlap) {
@@ -602,30 +626,28 @@ static int integrate_frame(b2v_volume *v, const float *depth, const uint8_t *col
     if (pe) B2V_CUDA(v, cudaEventRecord(pe[3], cs));
     if (v->overlap) B2V_CUDA(v, cudaEventRecord(v->ev_int_done[ring], cs));
     v->launches += 1;
-    if (v->prof_enabled) v->prof_int_launches += 1;
     return B2V_OK;
 }
 
 extern "C" int b2v_integrate(b2v_volume *v, const float *depth, const uint8_t *color, int32_t height,
                              int32_t width, const double K[4], const double Tcw[16], void *stream) {
     if (!v) return B2V_ERR_INVALID_ARGUMENT;
-    return integrate_frame(v, depth, color, height, width, K, Tcw, stream);
+    FrameImages in{{depth, 0.0f}, color, height, width};
+    const int rc = check_integrate(v, "b2v_integrate", false, 1, &in, K, Tcw, stream);
+    return rc != B2V_OK ? rc : integrate_frame(v, in, 0, K, Tcw, stream);
 }
 
 extern "C" int b2v_set_rectification(b2v_volume *v, const float *map_x, const float *map_y, int32_t height,
                                      int32_t width, int32_t swap_rb) {
     if (!v) return B2V_ERR_INVALID_ARGUMENT;
-    const int rc = read_counters(v);  // drains every stream
-    if (rc == B2V_ERR_CUDA) return rc;
+    B2V_CUDA(v, cudaSetDevice(v->cfg.device));
+    B2V_CUDA(v, cudaDeviceSynchronize());  // remap kernels on any stream may still read the maps and rectified slots
     cudaFree(v->d_mapx);
     cudaFree(v->d_mapy);
-    cudaFree(v->d_rdepth[0]);
-    cudaFree(v->d_rcolor[0]);
-    v->d_mapx = v->d_mapy = nullptr;
-    for (int s = 0; s < kStage; ++s) {
-        v->d_rdepth[s] = nullptr;
-        v->d_rcolor[s] = nullptr;
-    }
+    cudaFree(v->d_rdepth);
+    cudaFree(v->d_rcolor);
+    v->d_mapx = v->d_mapy = v->d_rdepth = nullptr;
+    v->d_rcolor = nullptr;  // ensure_staging allocates the rectified slots while maps are installed
     v->rect_H = v->rect_W = 0;
     v->rect_swap = swap_rb;
     v->map_cache.clear();
@@ -639,14 +661,6 @@ extern "C" int b2v_set_rectification(b2v_volume *v, const float *map_x, const fl
     B2V_CUDA(v, cudaMalloc(&v->d_mapy, pixels * sizeof(float)));
     B2V_CUDA(v, cudaMemcpy(v->d_mapx, map_x, pixels * sizeof(float), cudaMemcpyHostToDevice));
     B2V_CUDA(v, cudaMemcpy(v->d_mapy, map_y, pixels * sizeof(float), cudaMemcpyHostToDevice));
-    float *dbase = nullptr;
-    uint8_t *cbase = nullptr;
-    B2V_CUDA(v, cudaMalloc(&dbase, pixels * sizeof(float) * kStage));
-    B2V_CUDA(v, cudaMalloc(&cbase, pixels * 3 * kStage));
-    for (int s = 0; s < kStage; ++s) {
-        v->d_rdepth[s] = dbase + pixels * s;
-        v->d_rcolor[s] = cbase + pixels * 3 * s;
-    }
     v->rect_H = height;
     v->rect_W = width;
     return B2V_OK;
@@ -681,58 +695,13 @@ extern "C" int b2v_remap(const void *src, int32_t kind, int32_t height, int32_t 
     return e == cudaSuccess ? B2V_OK : B2V_ERR_CUDA;
 }
 
-// rectify one frame (raw staging or caller device buffers -> rectified slot), on the allocate stream
-static int rectify_frame(b2v_volume *v, const float **d_depth, const uint8_t **d_color, int H, int W, int slot,
-                         cudaStream_t as) {
-    if (!v->d_mapx) return B2V_OK;
-    if (H != v->rect_H || W != v->rect_W) {
-        v->err = "rectification maps were installed for a different image size";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    B2V_CUDA(v, launch_remap_b32_nearest(*d_depth, H, W, v->d_mapx, v->d_mapy, v->d_rdepth[slot], as));
-    B2V_CUDA(v, launch_remap_u8c3_linear(*d_color, H, W, v->d_mapx, v->d_mapy, v->d_rcolor[slot], v->rect_swap, as));
-    *d_depth = v->d_rdepth[slot];
-    *d_color = v->d_rcolor[slot];
-    v->launches += 2;
-    return B2V_OK;
-}
-
-static int ensure_group_buffers(b2v_volume *v, size_t pixels) {
-    if (pixels <= v->gtex_pixels) return B2V_OK;
-    B2V_CUDA(v, cudaDeviceSynchronize());
-    v->gtex_pixels = 0;  // stays 0 if an allocation below fails
-    for (float4 *&t : v->d_gtex) {
-        cudaFree(t);
-        t = nullptr;
-        B2V_CUDA(v, cudaMalloc(&t, pixels * sizeof(float4)));
-    }
-    v->gtex_pixels = pixels;
-    return B2V_OK;
-}
-
-extern "C" int b2v_integrate_batch(b2v_volume *v, int32_t n_frames, const float *depth,
-                                   const uint8_t *color, int32_t height, int32_t width,
-                                   const double K[4], const double *Tcw, void *stream) {
-    if (!v) return B2V_ERR_INVALID_ARGUMENT;
-    if (n_frames < 0 || (n_frames > 0 && (!depth || !color || !Tcw || !K)) || height <= 0 || width <= 0) {
-        v->err = "b2v_integrate_batch: bad arguments";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    if (n_frames == 0) return B2V_OK;
-    if (!(K[0] > 0.0) || !(K[1] > 0.0)) {
-        v->err = "b2v_integrate_batch: focal lengths must be positive";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    B2V_CUDA(v, cudaSetDevice(v->cfg.device));
-    const size_t pixels = static_cast<size_t>(height) * width;
-    const bool dd = is_device_pointer(depth), dc = is_device_pointer(color);
-    const int dev_hint = dd == dc ? (dd ? 1 : 0) : -1;
-    if (stream != nullptr && dev_hint != 1) {
-        v->err = "b2v_integrate_batch: a caller stream requires device image pointers";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
+// the frames of `in` in fused groups of group_frames: per group, the uploads, ONE allocate_group launch and ONE
+// integrate_group launch (frame by frame when fusion is off)
+static int integrate_batch(b2v_volume *v, int32_t n_frames, const FrameImages &in, const double K[4],
+                           const double *Tcw, void *stream) {
     cudaStream_t cs = stream ? static_cast<cudaStream_t>(stream) : v->compute;
     cudaStream_t as = v->overlap ? v->alloc : cs;
+    const bool dev_inputs = in.dev_depth && in.dev_color;
     struct FenceGuard {  // every exit path (errors included) drops the batch-wide input fence
         b2v_volume *v;
         ~FenceGuard() { v->inputs_fenced = false; }
@@ -742,38 +711,33 @@ extern "C" int b2v_integrate_batch(b2v_volume *v, int32_t n_frames, const float 
         // producers, earlier per-frame work) happens before the batch's allocate kernels.  A caller that knows better
         // (b2v_set_input_event: "the inputs are ready when this event fires") keeps the allocate kernels of this batch
         // from also waiting for the update kernels of the previous one.
-        if (v->input_event && dev_hint == 1) {
+        if (v->input_event && dev_inputs) {
             B2V_CUDA(v, cudaStreamWaitEvent(v->alloc, v->input_event, 0));
         } else {
             B2V_CUDA(v, cudaEventRecord(v->ev_in, cs));
             B2V_CUDA(v, cudaStreamWaitEvent(v->alloc, v->ev_in, 0));
         }
         v->inputs_fenced = true;
-    } else if (v->input_event && dev_hint == 1) {
+    } else if (v->input_event && dev_inputs) {
         B2V_CUDA(v, cudaStreamWaitEvent(cs, v->input_event, 0));
     }
     v->input_event = nullptr;
     int rc = B2V_OK;
-    const bool u16 = v->in_u16_scale > 0.0f;  // `depth` is really const uint16_t *
-    const uint16_t *depth16 = reinterpret_cast<const uint16_t *>(depth);
     if (!v->fuse || n_frames < 2) {
         for (int32_t f = 0; f < n_frames && rc == B2V_OK; ++f)
-            rc = integrate_frame(v, u16 ? reinterpret_cast<const float *>(depth16 + pixels * f) : depth + pixels * f,
-                                 color + pixels * 3 * f, height, width, K, Tcw + 16 * static_cast<size_t>(f), stream,
-                                 dev_hint);
+            rc = integrate_frame(v, in, f, K, Tcw + 16 * static_cast<size_t>(f), stream);
         return rc;
     }
-    rc = ensure_group_buffers(v, pixels);
-    if (rc == B2V_OK) rc = ensure_staging(v, pixels);
-    if (rc == B2V_OK && u16) rc = ensure_staging16(v, pixels);
+    const size_t pixels = static_cast<size_t>(in.H) * in.W;
+    rc = ensure_staging(v, pixels, in.depth.u16_scale > 0.0f, true);
     if (rc != B2V_OK) return rc;
     v->rings_stale = true;
     v->last_stream = stream ? cs : nullptr;
-    const bool staged = dev_hint != 1;
     const int gsz = std::max(1, std::min(v->group_frames, kMaxGroup));
     for (int32_t g0 = 0; g0 < n_frames; g0 += gsz) {
         const int count = std::min<int32_t>(gsz, n_frames - g0);
         const int buf = static_cast<int>(v->group_id % kGroupBufs);
+        const int s0 = buf * kMaxGroup;
         // the group buffer (masks, union list, texel images) was last used by group id - kGroupBufs
         B2V_CUDA(v, cudaStreamWaitEvent(as, v->ev_group_done[buf], 0));
         B2V_CUDA(v, cudaMemsetAsync(v->meta.counters + group_ctr(buf, 0), 0, kGroupCtrStride * sizeof(uint32_t), as));
@@ -784,76 +748,35 @@ extern "C" int b2v_integrate_batch(b2v_volume *v, int32_t n_frames, const float 
         args.count = count;
         aargs.count = count;
         aargs.use_tma = 1;
-        if (staged) {
-            // the raw staging slots of this buffer were consumed by the allocate launch of group id - kGroupBufs;
-            // the group's frames are contiguous on both sides: one H2D copy per image type
-            B2V_CUDA(v, cudaStreamWaitEvent(v->copy, v->ev_galloc[buf], 0));
-            const int s0 = buf * kMaxGroup;
-            if (u16)
-                B2V_CUDA(v, cudaMemcpyAsync(v->d_depth16[s0], depth16 + pixels * g0, pixels * sizeof(uint16_t) * count,
-                                            cudaMemcpyHostToDevice, v->copy));
-            else
-                B2V_CUDA(v, cudaMemcpyAsync(v->d_depth[s0], depth + pixels * g0, pixels * sizeof(float) * count,
-                                            cudaMemcpyHostToDevice, v->copy));
-            B2V_CUDA(v, cudaMemcpyAsync(v->d_color[s0], color + pixels * 3 * g0, pixels * 3 * count,
-                                        cudaMemcpyHostToDevice, v->copy));
-        }
         for (int k = 0; k < count; ++k) {
-            const size_t f = static_cast<size_t>(g0 + k);
-            const float *d_depth = u16 ? nullptr : depth + pixels * f;
-            const uint8_t *d_color = color + pixels * 3 * f;
-            if (staged || u16) d_depth = v->d_depth[buf * kMaxGroup + k];  // (widened) float staging slot
-            if (staged) d_color = v->d_color[buf * kMaxGroup + k];
             FrameParams P;
-            fill_frame_params(&P, K, Tcw + 16 * f, height, width, v->geo, v->frame_id + 1);
+            fill_frame_params(&P, K, Tcw + 16 * static_cast<size_t>(g0 + k), in.H, in.W, v->geo, v->frame_id + 1);
             P.group_bit = k;
             P.group_buf = buf;
             aargs.pose[k] = P.pose;
             if (k == 0) {
                 aargs.P = P;
                 aargs.frame_id0 = v->frame_id + 1;
+                rc = refresh_lambda(v, P, K, in.H, in.W, as);
+                if (rc != B2V_OK) return rc;
             }
-            if (k == 0 && (v->lam_H != height || v->lam_W != width || std::memcmp(v->lam_K, K, sizeof(v->lam_K)) != 0)) {
-                if (v->overlap) B2V_CUDA(v, cudaStreamSynchronize(v->alloc));
-                B2V_CUDA(v, launch_lambda(P, v->d_lambda, as));
-                std::memcpy(v->lam_K, K, sizeof(v->lam_K));
-                v->lam_H = height;
-                v->lam_W = width;
-                v->launches += 1;
-            }
-            float4 *tex = v->d_gtex[buf * kMaxGroup + k];
-            aargs.depth[k] = d_depth;
-            aargs.color[k] = d_color;
+            float4 *tex = v->staged(v->d_gtex, s0, pixels, k);
             aargs.tex[k] = tex;
             P.I.tex = tex;
             args.f[k] = P.I;
             v->frame_id += 1;
         }
-        if (staged) {
-            B2V_CUDA(v, cudaEventRecord(v->ev_ready[buf], v->copy));  // all frames of the group uploaded
-            B2V_CUDA(v, cudaStreamWaitEvent(as, v->ev_ready[buf], 0));
-        }
-        if (u16) {  // widen the group's raw depth into its (contiguous) float staging slots in one launch
-            const uint16_t *src = staged ? v->d_depth16[buf * kMaxGroup] : depth16 + pixels * g0;
-            B2V_CUDA(v, launch_depth_u16_to_f32(src, v->d_depth[buf * kMaxGroup], pixels * count, v->in_u16_scale, as));
-            v->launches += 1;
-        }
-        for (int k = 0; k < count; ++k) {  // optional rectification, then the TMA descriptors of the final images
-            const int rrc = rectify_frame(v, &aargs.depth[k], &aargs.color[k], height, width, buf * kMaxGroup + k, as);
-            if (rrc != B2V_OK) return rrc;
-            const FrameMaps *fm = frame_maps(v, aargs.depth[k], aargs.color[k], height, width);
+        // the raw slots of this buffer were consumed by the allocate launch of group id - kGroupBufs
+        rc = prepare_frames(v, in, g0, count, s0, v->ev_galloc[buf], v->ev_ready[buf], as, aargs.depth, aargs.color);
+        if (rc != B2V_OK) return rc;
+        for (int k = 0; k < count; ++k) {  // the TMA descriptors of the final images
+            const FrameMaps *fm = frame_maps(v, aargs.depth[k], aargs.color[k], in.H, in.W);
             if (fm) aargs.maps[k] = *fm; else aargs.use_tma = 0;
         }
-        cudaEvent_t *pe = nullptr;
-        if (v->prof_enabled) {
-            const int prc = grow_profile_events(v, 4);
-            if (prc != B2V_OK) return prc;
-            pe = &v->prof_events[v->prof_used];
-            v->prof_used += 4;
-            v->prof_frames += count;
-            v->prof_int_launches += 1;
-            B2V_CUDA(v, cudaEventRecord(pe[0], as));
-        }
+        cudaEvent_t *pe;
+        rc = profile_events(v, count, &pe);
+        if (rc != B2V_OK) return rc;
+        if (pe) B2V_CUDA(v, cudaEventRecord(pe[0], as));
         aargs.lmap = v->lam_map;
         B2V_CUDA(v, launch_allocate_group(aargs, v->d_lambda, v->table, v->meta, as));
         if (pe) B2V_CUDA(v, cudaEventRecord(pe[1], as));
@@ -871,6 +794,15 @@ extern "C" int b2v_integrate_batch(b2v_volume *v, int32_t n_frames, const float 
     return B2V_OK;
 }
 
+extern "C" int b2v_integrate_batch(b2v_volume *v, int32_t n_frames, const float *depth,
+                                   const uint8_t *color, int32_t height, int32_t width,
+                                   const double K[4], const double *Tcw, void *stream) {
+    if (!v) return B2V_ERR_INVALID_ARGUMENT;
+    FrameImages in{{depth, 0.0f}, color, height, width};
+    const int rc = check_integrate(v, "b2v_integrate_batch", false, n_frames, &in, K, Tcw, stream);
+    return rc != B2V_OK || n_frames == 0 ? rc : integrate_batch(v, n_frames, in, K, Tcw, stream);
+}
+
 // Raw 16-bit depth (e.g. TUM / ScanNet PNGs): uploaded as uint16 (2 instead of 4 bytes per pixel over PCIe) and
 // widened on the device to float(u16) * depth_scale in float32 - the value numpy's
 // `depth.astype(np.float32) * depth_factor` produces (volumetric_integrator_base.py:1008-1015).
@@ -878,29 +810,18 @@ extern "C" int b2v_integrate_batch_u16(b2v_volume *v, int32_t n_frames, const ui
                                        const uint8_t *color, int32_t height, int32_t width, const double K[4],
                                        const double *Tcw, void *stream) {
     if (!v) return B2V_ERR_INVALID_ARGUMENT;
-    if (!(depth_scale > 0.0f)) {
-        v->err = "b2v_integrate_batch_u16: depth_scale must be positive";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    v->in_u16_scale = depth_scale;
-    const int rc = b2v_integrate_batch(v, n_frames, reinterpret_cast<const float *>(depth), color, height, width, K,
-                                       Tcw, stream);
-    v->in_u16_scale = 0.0f;
-    return rc;
+    FrameImages in{{depth, depth_scale}, color, height, width};
+    const int rc = check_integrate(v, "b2v_integrate_batch_u16", true, n_frames, &in, K, Tcw, stream);
+    return rc != B2V_OK || n_frames == 0 ? rc : integrate_batch(v, n_frames, in, K, Tcw, stream);
 }
 
 extern "C" int b2v_integrate_u16(b2v_volume *v, const uint16_t *depth, float depth_scale, const uint8_t *color,
                                  int32_t height, int32_t width, const double K[4], const double Tcw[16],
                                  void *stream) {
     if (!v) return B2V_ERR_INVALID_ARGUMENT;
-    if (!(depth_scale > 0.0f)) {
-        v->err = "b2v_integrate_u16: depth_scale must be positive";
-        return B2V_ERR_INVALID_ARGUMENT;
-    }
-    v->in_u16_scale = depth_scale;
-    const int rc = integrate_frame(v, reinterpret_cast<const float *>(depth), color, height, width, K, Tcw, stream);
-    v->in_u16_scale = 0.0f;
-    return rc;
+    FrameImages in{{depth, depth_scale}, color, height, width};
+    const int rc = check_integrate(v, "b2v_integrate_u16", true, 1, &in, K, Tcw, stream);
+    return rc != B2V_OK ? rc : integrate_frame(v, in, 0, K, Tcw, stream);
 }
 
 extern "C" int b2v_set_input_event(b2v_volume *v, void *event) {
@@ -987,17 +908,6 @@ extern "C" int b2v_profile_read(b2v_volume *v, double *allocate_ms, double *inte
     if (!v) return B2V_ERR_INVALID_ARGUMENT;
     B2V_CUDA(v, cudaSetDevice(v->cfg.device));
     double a = 0.0, b = 0.0;
-    if (std::getenv("B2V_DEBUG_TIMELINE") && v->prof_used >= 4) {  // debug: event times relative to the first
-        for (size_t k = 0; k + 3 < v->prof_used && k < 4 * 12; k += 4) {
-            float t[4];
-            for (int j = 0; j < 4; ++j) {
-                cudaEventSynchronize(v->prof_events[k + j]);
-                cudaEventElapsedTime(&t[j], v->prof_events[0], v->prof_events[k + j]);
-            }
-            std::fprintf(stderr, "[b2v timeline] launch %zu: alloc %.1f..%.1f us  integrate %.1f..%.1f us\n", k / 4,
-                         1e3 * t[0], 1e3 * t[1], 1e3 * t[2], 1e3 * t[3]);
-        }
-    }
     for (size_t k = 0; k + 3 < v->prof_used; k += 4) {
         B2V_CUDA(v, cudaEventSynchronize(v->prof_events[k + 1]));
         B2V_CUDA(v, cudaEventSynchronize(v->prof_events[k + 3]));

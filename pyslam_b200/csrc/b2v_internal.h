@@ -56,7 +56,7 @@ struct VolumeConsts {
 
 // Fused group integration: up to kMaxGroup consecutive frames are applied to a block while it is
 // resident in registers.
-constexpr int kMaxGroup = 32;   // frames per fused group (bits of the membership mask); the default group is 8
+constexpr int kMaxGroup = 32;   // frames per fused group (bits of the membership mask); the default group is 16
 // group state (masks, union list, texel images, counters) is kGroupBufs-deep: the allocation of group g+3 may
 // run while group g is still being integrated
 constexpr int kGroupBufs = 4;

@@ -1,6 +1,5 @@
 """Per-rank timing of an N-way hash-sharded job on ONE GPU (ranks share nothing, so rank 0 of N does that job's
-per-rank work): frames/s, period per group of 8 frames, and - with B2V_DEBUG_TIMELINE=1 - the start/end times of
-the allocate / integrate launches of the first groups.  Usage: python tools/shard_timeline.py [N]   (DESIGN.md §7)"""
+per-rank work): frames/s and period per group of 8 frames.  Usage: python tools/shard_timeline.py [N]   (DESIGN.md §7)"""
 import os, sys, time, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from pyslam_b200 import B200TsdfVolume
