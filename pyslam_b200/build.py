@@ -15,7 +15,7 @@ _DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_DIR, "csrc")
 LIB = os.path.join(_DIR, "libb2v.so")
 SOURCES = ["b2v_api.cu", "b2v_tsdf.cu", "b2v_mesh.cu", "b2v_grid.cu", "b2v_prep.cu", "b2v_semantic.cu"]
-HEADERS = ["b2v_device.cuh", "b2v_internal.h", "b2v_scan.cuh", "mc_tables.h", "../../include/b2v.h"]
+HEADERS = ["b2v_device.cuh", "b2v_internal.h", "b2v_points.cuh", "b2v_scan.cuh", "mc_tables.h", "../../include/b2v.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

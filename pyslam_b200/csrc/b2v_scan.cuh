@@ -1,5 +1,5 @@
 // b2v_scan.cuh — single-CTA exclusive scan over per-block counts (n <= a few million entries).
-// Used by the count -> scan -> emit passes of the mesher and of get_voxels.
+// Used by the count -> scan -> emit passes of the mesher and of the point grids' read-outs.
 #pragma once
 
 #include <cstdint>
@@ -121,6 +121,19 @@ scan_apply_kernel(const uint32_t *__restrict__ in_all, uint32_t *__restrict__ ou
     const uint32_t incl = x + (wid ? s_warp[wid - 1] : 0u);
     if (i < n) out[i] = prefix + incl - v;
     if (blockIdx.x == gridDim.x - 1 && t == 1023) totals[blockIdx.y] = prefix + incl;
+}
+
+// sums[blockIdx.x] = the number of threads of a 512-thread CTA that pass `keep`; s_warp: 16 words
+static __device__ __forceinline__ void block_count_512(bool keep, uint32_t *s_warp, uint32_t *sums) {
+    const int t = threadIdx.x;
+    const uint32_t x = __reduce_add_sync(0xffffffffu, keep ? 1u : 0u);
+    if ((t & 31) == 0) s_warp[t >> 5] = x;
+    __syncthreads();
+    if (t == 0) {
+        uint32_t s = 0;
+        for (int k = 0; k < 16; ++k) s += s_warp[k];
+        sums[blockIdx.x] = s;
+    }
 }
 
 // block-wide exclusive scan of one value per thread for a 512-thread CTA; s_warp: 16 words
