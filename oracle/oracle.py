@@ -327,6 +327,9 @@ def _o3d():
         L.o3d_dump_blocks.argtypes = [vp, vp, vp]
         L.o3d_extract_mesh.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.o3d_mesh_copy.argtypes = [_f64p, _f64p, _i32p, _i32p]
+        L.o3d_set_block.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, _f32p]
+        L.o3d_extract_point_cloud.argtypes = [vp, C.POINTER(C.c_int64)]
+        L.o3d_points_copy.argtypes = [_f64p, _f64p]
         _o3d_lib = L
     return _o3d_lib
 
@@ -395,6 +398,23 @@ class Open3DOrderVolume:
         T = np.zeros((nt.value, 3), np.int32)
         self._L.o3d_mesh_copy(V.reshape(-1), Cc.reshape(-1), E.reshape(-1), T.reshape(-1))
         return dict(vertices=V, colors=Cc, edges=E, triangles=T)
+
+    def set_blocks(self, keys, vox):
+        """Seed blocks in the product's layout (keys int32 [n,3], vox float32 [n,5,512]), e.g. a GPU volume's
+        `dump_blocks()`: each goes to its place in unit floor(key / (R/8)); the unit's other voxels keep weight 0."""
+        k = np.ascontiguousarray(keys, np.int32).reshape(-1, 3)
+        v = np.ascontiguousarray(vox, np.float32).reshape(k.shape[0], 5 * 512)
+        for key, block in zip(k, v):
+            self._L.o3d_set_block(self._h, int(key[0]), int(key[1]), int(key[2]), block)
+
+    def extract_point_cloud(self):
+        """ScalableTSDFVolume::ExtractPointCloud: points and colours float64 [n,3], in Open3D's loop order."""
+        n = C.c_int64(0)
+        self._L.o3d_extract_point_cloud(self._h, C.byref(n))
+        P = np.zeros((n.value, 3), np.float64)
+        Cc = np.zeros((n.value, 3), np.float64)
+        self._L.o3d_points_copy(P.reshape(-1), Cc.reshape(-1))
+        return dict(points=P, colors=Cc)
 
 
 def canonical_mesh(vertices, colors, edges, triangles):
